@@ -1,4 +1,4 @@
-"""The UNMODIFIED reference (astooke/rlpyt, installed into baseline/_ref by the recipe in DESIGN.md section 5)
+"""The UNMODIFIED reference (astooke/rlpyt, copied into oracle/_ref by oracle/reference_install.py)
 driven through its own public API for bench.py's ``--impl reference`` arm:
 
     GpuSampler(EnvCls, batch_T, batch_B).initialize(agent, affinity, seed, bootstrap_value)
@@ -12,19 +12,15 @@ path; the only thing supplied is the synthetic Atari-shaped environment (``atari
 there is no network), written against the reference's ``Env`` interface with the same behaviour as
 rlpyt_b200/envs/synthetic.py.
 """
-import os
 import sys
 import time
 from collections import namedtuple
 
 import numpy as np
 
-REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
+from oracle.reference_install import DEST as REF, available  # noqa: F401
+
 EnvInfo = namedtuple("EnvInfo", ["game_score", "traj_done"])     # module level: the reference pickles an example
-
-
-def available():
-    return os.path.isdir(os.path.join(REF, "rlpyt"))
 
 
 def _import():

@@ -2,6 +2,7 @@
 """bench.py - the driver's measurement contract.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload ppo|gae|replay|dqn]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -145,7 +146,9 @@ def run_b200(args):
     affinity = make_affinity(local_rank, args.workers or None, local_rank=local_rank, ranks_per_node=world,
                              node_share=8, smt_workers=args.workers_per_core >= 2)
     if sampler_kind == "alternating" and len(affinity["workers_cpus"]) % 2:
-        affinity["workers_cpus"] = affinity["workers_cpus"][:-1] or affinity["workers_cpus"]
+        # two equal worker groups: drop the odd worker; a share with one worker core runs one worker per group on it
+        wc = affinity["workers_cpus"]
+        affinity["workers_cpus"] = wc[:-1] if len(wc) > 1 else wc * 2
     n_workers = len(affinity["workers_cpus"])
     sampler.initialize(agent, affinity=affinity, seed=seed + 1, bootstrap_value=True, world_size=world, rank=rank)
     agent.to_device(local_rank)
@@ -177,6 +180,7 @@ def run_b200(args):
             barrier()
         t_value = max_over_ranks(e0.elapsed_time(e1) * 1e-3)
         launches = _lib.launch_count - l0
+        dumps = step_outputs("learner", info, agent) if args.dump_outputs else {}
         value = steps_per_itr * K / t_value
         # device time of the returns + loss kernels INSIDE a real optimize_agent iteration (CUDA events around
         # process_returns and around each fused-loss call; the stream is kept busy by the network kernels, so the
@@ -213,6 +217,8 @@ def run_b200(args):
                 itr += 1
             barrier()
             t_e2e = max_over_ranks(time.perf_counter() - t0)
+        if args.dump_outputs:
+            dumps.update(step_outputs("e2e", info, agent, samples))
         e2e = steps_per_itr * K / t_e2e
         sampler_profile = None
         pr = getattr(sampler, "profile", None)
@@ -286,7 +292,51 @@ def run_b200(args):
         dist.barrier()
         dist.destroy_process_group()
     if rank == 0:
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, dumps)
         print(json.dumps(out), flush=True)
+
+
+DUMP_FRAMES = 16         # whole observation frames in the dump, drawn with a fixed seed from the [T,B] batch
+DUMP_LIMIT = 64 << 20    # bytes
+
+
+def _f(x):
+    """Host copy as float32 / float64; integer and boolean arrays become float64 (exact)."""
+    a = x.detach().cpu().numpy() if torch.is_tensor(x) else np.asarray(x)
+    return a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+
+
+def step_outputs(prefix, info, agent, samples=None):
+    """What the last step of a timed loop handed its caller: ``optimize_agent``'s OptInfo rows and the parameters
+    it updated, and for the end-to-end loop the batch ``obtain_samples`` returned.  The batch's observations
+    (925 MB of frames) enter as every frame's byte sum plus DUMP_FRAMES whole frames."""
+    out = {f"{prefix}_info_{k}": np.asarray(getattr(info, k), np.float64) for k in info._fields}
+    out.update({f"{prefix}_param_{k}": _f(v) for k, v in agent.state_dict().items()})
+    if samples is not None:
+        a, e = samples.agent, samples.env
+        obs = e.observation
+        T, B = obs.shape[:2]
+        pick = np.random.default_rng(0).choice(T * B, DUMP_FRAMES, replace=False)
+        rows = torch.as_tensor(pick, device=obs.device)
+        out.update({
+            f"{prefix}_action": _f(a.action), f"{prefix}_prev_action": _f(a.prev_action),
+            f"{prefix}_prob": _f(a.agent_info.dist_info.prob), f"{prefix}_value": _f(a.agent_info.value),
+            f"{prefix}_bootstrap_value": _f(a.bootstrap_value), f"{prefix}_reward": _f(e.reward),
+            f"{prefix}_prev_reward": _f(e.prev_reward), f"{prefix}_done": _f(e.done),
+            f"{prefix}_observation_sum": _f(obs.sum(dim=tuple(range(2, obs.dim())), dtype=torch.float64)),
+            f"{prefix}_observation_frames": obs.reshape(T * B, *obs.shape[2:])[rows].float().cpu().numpy(),
+            f"{prefix}_observation_frame_index": pick.astype(np.float64)})
+    return out
+
+
+def write_outputs(path, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT} byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def roofline_gae(U, T=128, B=1 << 20, reps=10):
@@ -461,7 +511,7 @@ def step_kernel_rooflines(N=8192, reps=10):
 
 
 def cpu_baseline(U):
-    """Rank 0, N=1: (i) the reference arm (``--impl reference``: the unmodified reference from baseline/_ref on
+    """Rank 0, N=1: (i) the reference arm (``--impl reference``: the unmodified reference from oracle/_ref on
     this box's host cores, bounded sample, same config) run as a child process for a few steps - its line's
     ``value`` (learner only) and ``e2e`` (sampler + learner) are what ``value`` / ``e2e`` above compare with;
     (ii) the north_star unit "reference CPU GAE + PPO-loss" at [128,256] (GAE on torch-CPU tensors + 16 x loss
@@ -555,14 +605,14 @@ def _reference_affinity(world):
 
 
 def run_reference(args):
-    """``--impl reference``: the UNMODIFIED reference (baseline/_ref, installed by the pip recipe in DESIGN.md
-    section 5) through its own API - ``GpuSampler`` with ``cuda_idx=None`` (batched action serving on torch-CPU
+    """``--impl reference``: the UNMODIFIED reference (oracle/_ref, copied there by oracle/reference_install.py)
+    through its own API - ``GpuSampler`` with ``cuda_idx=None`` (batched action serving on torch-CPU
     with every host thread, env stepping in forked workers pinned to the same cores this repo's arm uses) +
     ``PPO.optimize_agent`` on torch-CPU - baseline/reference_arm.py.  Same config as the b200 arm (B=256, the
     same PPO hyper-parameters, env and worker cores); each step is a bounded sample [T=16, B=256] of the
     [T=128, B=256] iteration (4096 of 32768 env-steps: per-env-step cost does not depend on T).
     ``value`` = learner only (optimize_agent), ``e2e`` = sampler + learner: like for like with the b200 line.
-    Falls back to the oracle port when baseline/_ref is absent."""
+    Falls back to the oracle port when oracle/_ref is absent."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -588,7 +638,7 @@ def run_reference(args):
         loop.shutdown()
     steps = REF_T * B_CFG
     val_e2e, val_learn = steps * K / dt, steps * K / t_opt
-    sample = (f"unmodified reference (baseline/_ref): GpuSampler(cuda_idx=None, {len(workers_cpus)} worker processes) + "
+    sample = (f"unmodified reference (oracle/_ref): GpuSampler(cuda_idx=None, {len(workers_cpus)} worker processes) + "
               f"PPO on torch-CPU fp32, {threads} threads; bounded sample [T={REF_T},B={B_CFG}] per step "
               f"({steps} of {T_CFG * B_CFG} env-steps), minibatches=4 epochs=4")
     out = {
@@ -633,7 +683,7 @@ def run_reference(args):
 
 
 def run_reference_port(args):
-    """Fallback when baseline/_ref is missing: the oracle port (serial CPU rollout + PPO on torch-CPU)."""
+    """Fallback when oracle/_ref is missing: the oracle port (serial CPU rollout + PPO on torch-CPU)."""
     from oracle import atari_ff
     from oracle.collector import SerialRollout
     from oracle.ppo import PpoOracle
@@ -666,7 +716,7 @@ def run_reference_port(args):
         step(W + i)
     dt = time.perf_counter() - t0
     val = Tb * Bb * K / dt
-    sample = (f"oracle port (serial collector + PPO, torch-CPU fp32, {threads} threads; baseline/_ref missing), bounded sample "
+    sample = (f"oracle port (serial collector + PPO, torch-CPU fp32, {threads} threads; oracle/_ref missing), bounded sample "
               f"[T={Tb},B={Bb}] per step ({Tb * Bb} of {T_CFG * B_CFG} env-steps)")
     print(json.dumps({
         "impl": "reference", "metric": "env-steps/sec PPO Atari [T=128,B=256] at 1/2/4/8 GPU; GAE-scan GB/s",
@@ -692,7 +742,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-context", action="store_true", help="reference arm: skip the stock-PyTorch-on-GPU context leg")
     ap.add_argument("--workload", default="ppo", choices=["ppo", "gae", "replay", "dqn"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last step of each timed loop computed to DIR/<name>.npy (ppo workload, b200 arm)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.workload != "ppo" or args.impl != "b200"):
+        ap.error("--dump-outputs is implemented for the ppo workload of the b200 arm")
     if args.workload != "ppo":
         from tools import workload_benches
         return workload_benches.run(args)

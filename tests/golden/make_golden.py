@@ -837,8 +837,90 @@ def gen_collector():
     _save("collector", out)
 
 
+def gen_live_reference():
+    """The reference's outputs on the seeded random cases of tests/live_reference_cases.py: returns, PPO loss,
+    DQN loss (with gradients) and sum-tree op sequences."""
+    from collections import namedtuple
+    import torch
+    sys.path.insert(0, os.path.dirname(HERE))                     # tests/
+    import live_reference_cases as C
+    from rlpyt.agents.base import AgentInputs
+    from rlpyt.algos import utils as R
+    from rlpyt.algos.dqn.dqn import DQN
+    from rlpyt.algos.pg.ppo import PPO
+    from rlpyt.distributions.categorical import Categorical, DistInfo
+    from rlpyt.replays.sum_tree import SumTree
+    out = {}
+    for seed in C.RETURNS_SEEDS:
+        c, pre = C.returns_case(seed), f"returns/{seed}/"
+        done_f = c["done"].astype(np.float32)
+        out[pre + "adv"], out[pre + "ret"] = R.generalized_advantage_estimation(c["reward"], c["value"], done_f, c["bv"],
+                                                                              c["gamma"], c["lam"])
+        out[pre + "discount_return"] = R.discount_return(c["reward"], done_f, c["bv"], c["gamma"])
+        out[pre + "valid"] = R.valid_from_done(torch.from_numpy(done_f)).numpy()
+        nstep = [R.discount_return_n_step(c["reward"], c["done"], n, c["gamma"], do_truncated=trunc)
+                 for n, trunc in c["n_steps"]]
+        out[pre + "nstep_shape"] = np.array([r.shape for r, _ in nstep], np.int64)   # truncated returns are shorter
+        out[pre + "nstep_return"] = np.concatenate([r.ravel() for r, _ in nstep])
+        out[pre + "nstep_done"] = np.concatenate([d.ravel() for _, d in nstep])
+
+    class PgStub:
+        recurrent = False
+
+        def __init__(self, p, v, dist):
+            self.p, self.v, self.distribution = p, v, dist
+
+        def __call__(self, observation, prev_action, prev_reward):
+            return DistInfo(prob=self.p), self.v
+
+    for seed in C.PG_SEEDS:
+        c, pre = C.pg_case(seed), f"pg/{seed}/"
+        N, A = c["p_new"].shape
+        p = torch.from_numpy(c["p_new"]).clone().requires_grad_(True)
+        v = torch.from_numpy(c["value"]).clone().requires_grad_(True)
+        algo = PPO(value_loss_coeff=c["c_v"], entropy_loss_coeff=c["c_ent"], ratio_clip=c["clip"])
+        algo.agent = PgStub(p, v, Categorical(dim=A))
+        z = torch.zeros(N)
+        loss, ent, perp = algo.loss(AgentInputs(z, z, z), torch.from_numpy(c["action"]), torch.from_numpy(c["ret"]),
+                                    torch.from_numpy(c["adv"]), None if c["valid"] is None else torch.from_numpy(c["valid"]),
+                                    DistInfo(prob=torch.from_numpy(c["p_old"])))
+        loss.backward()
+        out[pre + "loss_entropy_perplexity"] = np.array([loss.item(), ent.item(), perp.item()], np.float64)
+        out[pre + "grad_prob"], out[pre + "grad_value"] = p.grad.numpy(), v.grad.numpy()
+
+    S = namedtuple("S", "agent_inputs action return_ done done_n target_inputs is_weights")
+    for seed in C.DQN_SEEDS:
+        c, pre = C.dqn_case(seed), f"dqn/{seed}/"
+        N = len(c["action"])
+        q = torch.from_numpy(c["qs"]).clone().requires_grad_(True)
+
+        class Stub:
+            def __call__(self, observation, prev_action, prev_reward):
+                return q if int(observation[0]) == 0 else torch.from_numpy(c["nq"])
+
+            def target(self, observation, prev_action, prev_reward):
+                return torch.from_numpy(c["tq"])
+
+        algo = DQN(discount=c["discount"], delta_clip=c["clip"], n_step_return=c["n_step"], double_dqn=c["double"],
+                   prioritized_replay=c["pri"])
+        algo.mid_batch_reset, algo.agent = True, Stub()
+        z = torch.zeros(N)
+        loss, td = algo.loss(S(AgentInputs(z, z, z), torch.from_numpy(c["action"]), torch.from_numpy(c["ret"]),
+                               torch.from_numpy(c["done_n"]), torch.from_numpy(c["done_n"]), AgentInputs(z + 1, z, z),
+                               torch.from_numpy(c["isw"])))
+        loss.backward()
+        out[pre + "loss"] = np.array([loss.item()], np.float64)
+        out[pre + "td_abs_errors"], out[pre + "grad_qs"] = td.numpy(), q.grad.numpy()
+
+    for seed in C.SUM_TREE_SEEDS:
+        for k, x in C.sum_tree_trace(SumTree, seed).items():
+            out[f"sum_tree/{seed}/{k}"] = x
+    _save("live_reference", out)
+
+
 GROUPS = {"returns": gen_returns, "loss": gen_loss, "ppo": gen_ppo, "replay": gen_replay, "dqn": gen_dqn,
-          "collector": gen_collector, "ppo_lstm": gen_ppo_lstm, "seq_replay": gen_seq_replay, "r2d1": gen_r2d1}
+          "collector": gen_collector, "ppo_lstm": gen_ppo_lstm, "seq_replay": gen_seq_replay, "r2d1": gen_r2d1,
+          "live_reference": gen_live_reference}
 
 
 def main():

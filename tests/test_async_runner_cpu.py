@@ -40,7 +40,8 @@ class FakeSampler:
     def batch_size(self):
         return self.batch_spec.size
 
-    def async_initialize(self, agent, bootstrap_value=False, traj_info_kwargs=None, seed=None):
+    def async_initialize(self, agent, bootstrap_value=False, traj_info_kwargs=None, seed=None, device=None):
+        # ``device``: the runner passes its CUDA device where one exists; this stand-in stays on the host (self.device None)
         self.agent = agent
         self.traj_info_kwargs = traj_info_kwargs
         return self.double_buffer, dict(observation=np.zeros(3))

@@ -1,12 +1,11 @@
 """Drop-in proof (north_star: "existing runners ... drop in"): the UNMODIFIED reference runner
-``rlpyt.runners.minibatch_rl.MinibatchRl`` (from baseline/_ref, or /root/reference in the build container) drives
+``rlpyt.runners.minibatch_rl.MinibatchRl`` (from oracle/_ref, see oracle/reference_install.py) drives
 this repo's GpuSampler / AlternatingSampler + AtariFfAgent + PPO (and SerialSampler + A2C, BASELINE.json configs[0]
 plumbing) through its own ``startup()`` / ``train()``: sampler.initialize(agent, affinity, seed, bootstrap_value,
 traj_info_kwargs, rank, world_size) -> agent.to_device -> algo.initialize(agent, n_itr, batch_spec, mid_batch_reset,
 examples, world_size, rank) -> [sample_mode, obtain_samples, train_mode, optimize_agent, store/log diagnostics] x n
 -> shutdown (rlpyt/runners/minibatch_rl.py:52-96, 246-263).  Only ``pyprind`` (a progress bar the image does not
 have) is stubbed."""
-import os
 import sys
 import types
 
@@ -16,17 +15,13 @@ import torch
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
 
 def _reference_runner():
-    for cand in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.isdir(os.path.join(cand, "rlpyt")):
-            if cand not in sys.path:
-                sys.path.insert(0, cand)
-            break
-    else:
-        pytest.skip("the reference package is not available (baseline/_ref)")
+    from oracle import reference_install
+    if not reference_install.available():
+        pytest.skip("the reference package is not available (oracle/_ref was not built)")
+    if reference_install.DEST not in sys.path:
+        sys.path.insert(0, reference_install.DEST)
     if "pyprind" not in sys.modules:                      # rlpyt/utils/prog_bar.py:3
         stub = types.ModuleType("pyprind")
 

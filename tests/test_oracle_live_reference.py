@@ -1,164 +1,64 @@
-"""Property tests of the oracle against the UNMODIFIED reference imported live from /root/reference
-(build container only - skipped wherever the reference tree is absent, e.g. on the GPU box, where the
-committed golden vectors of tests/golden/ take over).  Random shapes / seeds beyond the golden cases:
-returns (bit-exact), PPO / A2C / DQN losses with gradients (bit-exact, same torch ops), sum-tree op
-sequences (bit-exact tree contents and samples)."""
+"""Property tests of the oracle against the UNMODIFIED reference on random shapes / seeds beyond the golden
+cases (tests/live_reference_cases.py; the reference's outputs are stored in tests/golden/live_reference.npz by
+``tests/golden/make_golden.py --only live_reference``): returns (bit-exact), PPO / A2C / DQN losses with
+gradients (bit-exact, same torch ops), sum-tree op sequences (bit-exact tree contents and samples)."""
 import os
 import sys
-import types
 
 import numpy as np
 import pytest
 import torch
 
-REF = os.environ.get("RLPYT_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "rlpyt")),
-                                reason="reference tree not present (GPU box): golden vectors cover parity")
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+import live_reference_cases as C  # noqa: E402
 
 
 @pytest.fixture(scope="module")
-def ref():
-    sys.dont_write_bytecode = True
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    if "pyprind" not in sys.modules:       # rlpyt.utils.prog_bar needs pyprind (absent): stub
-        stub = types.ModuleType("pyprind")
-        stub.ProgBar = type("ProgBar", (), {"__init__": lambda self, *a, **k: None,
-                                            "update": lambda self, *a, **k: None, "stop": lambda self: None})
-        sys.modules["pyprind"] = stub
-    import rlpyt  # noqa: F401
-    return True
+def ref(golden):
+    return golden("live_reference")
 
 
-@pytest.mark.parametrize("seed", range(8))
+@pytest.mark.parametrize("seed", C.RETURNS_SEEDS)
 def test_returns_random_shapes(ref, seed):
-    from rlpyt.algos import utils as R
     from oracle import returns as O
-    rng = np.random.default_rng(100 + seed)
-    T, B = int(rng.integers(1, 40)), int(rng.integers(1, 9))
-    reward = rng.standard_normal((T, B)).astype(np.float32)
-    value = rng.standard_normal((T, B)).astype(np.float32)
-    done = rng.random((T, B)) < 0.15
-    bv = rng.standard_normal((1, B)).astype(np.float32)
-    done_f = done.astype(np.float32)
-    gam, lam = float(rng.choice([0.99, 0.9, 1.0, 0.5])), float(rng.choice([1.0, 0.98, 0.95, 0.0]))
-    adv, ret = R.generalized_advantage_estimation(reward, value, done_f, bv, gam, lam)
+    c, pre = C.returns_case(seed), f"returns/{seed}/"
+    reward, value, done, bv, gam, lam = c["reward"], c["value"], c["done"], c["bv"], c["gamma"], c["lam"]
     o_adv, o_ret = O.generalized_advantage_estimation(reward, value, done, bv, gam, lam)
-    assert np.array_equal(adv, o_adv) and np.array_equal(ret, o_ret)
-    assert np.array_equal(R.discount_return(reward, done_f, bv, gam), O.discount_return(reward, done, bv, gam))
-    assert np.array_equal(R.valid_from_done(torch.from_numpy(done_f)).numpy(), O.valid_from_done(done))
-    for n in range(1, min(T, 5) + 1):
-        for trunc in (False, True):
-            r_, d_ = R.discount_return_n_step(reward, done, n, gam, do_truncated=trunc)
-            o_r, o_d = O.discount_return_n_step(reward, done, n, gam, do_truncated=trunc)
-            assert np.array_equal(r_, o_r) and np.array_equal(d_, o_d)
+    assert np.array_equal(ref[pre + "adv"], o_adv) and np.array_equal(ref[pre + "ret"], o_ret)
+    assert np.array_equal(ref[pre + "discount_return"], O.discount_return(reward, done, bv, gam))
+    assert np.array_equal(ref[pre + "valid"], O.valid_from_done(done))
+    nstep = [O.discount_return_n_step(reward, done, n, gam, do_truncated=trunc) for n, trunc in c["n_steps"]]
+    assert np.array_equal(ref[pre + "nstep_shape"], [r.shape for r, _ in nstep])
+    assert np.array_equal(ref[pre + "nstep_shape"], [d.shape for _, d in nstep])
+    assert np.array_equal(ref[pre + "nstep_return"], np.concatenate([r.ravel() for r, _ in nstep]))
+    assert np.array_equal(ref[pre + "nstep_done"], np.concatenate([d.ravel() for _, d in nstep]))
 
 
-class _PgStub:
-    recurrent = False
-
-    def __init__(self, p, v, dist):
-        self.p, self.v, self.distribution = p, v, dist
-
-    def __call__(self, observation, prev_action, prev_reward):
-        from rlpyt.distributions.categorical import DistInfo
-        return DistInfo(prob=self.p), self.v
-
-
-@pytest.mark.parametrize("seed", range(6))
+@pytest.mark.parametrize("seed", C.PG_SEEDS)
 def test_pg_losses_random(ref, seed):
-    from rlpyt.agents.base import AgentInputs
-    from rlpyt.algos.pg.ppo import PPO
-    from rlpyt.distributions.categorical import Categorical, DistInfo
     from oracle import pg_loss as L
-    rng = np.random.default_rng(200 + seed)
-    N, A = int(rng.integers(1, 300)), int(rng.integers(2, 19))
-    p_new = rng.dirichlet(np.ones(A), N).astype(np.float32)
-    p_old = rng.dirichlet(np.ones(A), N).astype(np.float32)
-    value, ret, adv = (rng.standard_normal(N).astype(np.float32) for _ in range(3))
-    action = rng.integers(0, A, N).astype(np.int64)
-    valid = (rng.random(N) < 0.8).astype(np.float32) if seed % 2 else None
-    if valid is not None:
-        valid[0] = 1.0
-    clip, c_v, c_ent = 0.1 + 0.1 * (seed % 3), 0.5 + 0.25 * seed, 0.01 * seed
-    p = torch.from_numpy(p_new).clone().requires_grad_(True)
-    v = torch.from_numpy(value).clone().requires_grad_(True)
-    algo = PPO(value_loss_coeff=c_v, entropy_loss_coeff=c_ent, ratio_clip=clip)
-    algo.agent = _PgStub(p, v, Categorical(dim=A))
-    z = torch.zeros(N)
-    loss, ent, perp = algo.loss(AgentInputs(z, z, z), torch.from_numpy(action), torch.from_numpy(ret),
-                                torch.from_numpy(adv), None if valid is None else torch.from_numpy(valid),
-                                DistInfo(prob=torch.from_numpy(p_old)))
-    loss.backward()
-    o = L.ppo_loss(p_new, value, p_old, action, ret, adv, valid, clip, c_v, c_ent)
-    assert [o["loss"], o["entropy"], o["perplexity"]] == [loss.item(), ent.item(), perp.item()]
-    assert np.array_equal(o["grad_prob"], p.grad.numpy()) and np.array_equal(o["grad_value"], v.grad.numpy())
+    c, pre = C.pg_case(seed), f"pg/{seed}/"
+    o = L.ppo_loss(c["p_new"], c["value"], c["p_old"], c["action"], c["ret"], c["adv"], c["valid"], c["clip"], c["c_v"],
+                   c["c_ent"])
+    assert [o["loss"], o["entropy"], o["perplexity"]] == ref[pre + "loss_entropy_perplexity"].tolist()
+    assert np.array_equal(o["grad_prob"], ref[pre + "grad_prob"]) and np.array_equal(o["grad_value"], ref[pre + "grad_value"])
 
 
-@pytest.mark.parametrize("seed", range(6))
+@pytest.mark.parametrize("seed", C.DQN_SEEDS)
 def test_dqn_loss_random(ref, seed):
-    from collections import namedtuple
-    from rlpyt.agents.base import AgentInputs
-    from rlpyt.algos.dqn.dqn import DQN
     from oracle.dqn_loss import dqn_loss
-    rng = np.random.default_rng(300 + seed)
-    N, A = int(rng.integers(1, 200)), int(rng.integers(2, 19))
-    qs, tq, nq = ((rng.standard_normal((N, A)) * 2).astype(np.float32) for _ in range(3))
-    action = rng.integers(0, A, N).astype(np.int64)
-    ret = rng.standard_normal(N).astype(np.float32)
-    done_n = rng.random(N) < 0.2
-    isw = (rng.random(N) * 0.9 + 0.1).astype(np.float32)
-    double, pri = bool(seed & 1), bool(seed & 2)
-    clip = [1.0, None, 0.25][seed % 3]
-    n_step, disc = 1 + seed % 4, [0.99, 0.9][seed % 2]
-    q = torch.from_numpy(qs).clone().requires_grad_(True)
-
-    class Stub:
-        def __call__(self, observation, prev_action, prev_reward):
-            return q if int(observation[0]) == 0 else torch.from_numpy(nq)
-
-        def target(self, observation, prev_action, prev_reward):
-            return torch.from_numpy(tq)
-
-    algo = DQN(discount=disc, delta_clip=clip, n_step_return=n_step, double_dqn=double, prioritized_replay=pri)
-    algo.mid_batch_reset, algo.agent = True, Stub()
-    S = namedtuple("S", "agent_inputs action return_ done done_n target_inputs is_weights")
-    z = torch.zeros(N)
-    loss, td = algo.loss(S(AgentInputs(z, z, z), torch.from_numpy(action), torch.from_numpy(ret),
-                           torch.from_numpy(done_n), torch.from_numpy(done_n), AgentInputs(z + 1, z, z),
-                           torch.from_numpy(isw)))
-    loss.backward()
+    c, pre = C.dqn_case(seed), f"dqn/{seed}/"
     t = torch.from_numpy
-    o_loss, o_td, o_grad = dqn_loss(t(qs), t(tq), t(nq) if double else None, t(action), t(ret), t(done_n),
-                                    t(isw) if pri else None, disc, n_step, clip)
-    assert float(o_loss) == loss.item()
-    assert np.array_equal(o_td.numpy(), td.numpy()) and np.array_equal(o_grad.numpy(), q.grad.numpy())
+    o_loss, o_td, o_grad = dqn_loss(t(c["qs"]), t(c["tq"]), t(c["nq"]) if c["double"] else None, t(c["action"]), t(c["ret"]),
+                                    t(c["done_n"]), t(c["isw"]) if c["pri"] else None, c["discount"], c["n_step"], c["clip"])
+    assert float(o_loss) == float(ref[pre + "loss"][0])
+    assert np.array_equal(o_td.numpy(), ref[pre + "td_abs_errors"]) and np.array_equal(o_grad.numpy(), ref[pre + "grad_qs"])
 
 
-@pytest.mark.parametrize("seed", range(5))
+@pytest.mark.parametrize("seed", C.SUM_TREE_SEEDS)
 def test_sum_tree_random_op_sequences(ref, seed):
-    from rlpyt.replays.sum_tree import SumTree as RefTree
     from oracle.sum_tree import SumTree
-    rng = np.random.default_rng(400 + seed)
-    T, B = int(rng.integers(12, 40)), int(rng.integers(1, 6))
-    off_b, off_f = int(rng.integers(1, 4)), int(rng.integers(1, 4))
-    dv = float(rng.choice([1.0, 0.5, 2.0]))
-    r, o = RefTree(T, B, off_b, off_f, default_value=dv), SumTree(T, B, off_b, off_f, default_value=dv)
-    for step in range(30):
-        adv = int(rng.integers(1, 5))
-        r.advance(adv)
-        o.advance(adv)
-        assert np.array_equal(r.tree, o.tree)
-        if o.tree[0] <= 0:
-            continue
-        n = int(rng.integers(1, 9))
-        unique = bool(step % 3 == 0) and 2 * n <= int((o.priorities > 0).sum())
-        np.random.seed(1000 * seed + step)               # both draw from the global numpy stream, like the reference
-        (rt, rb), rp = r.sample(n, unique=unique)
-        np.random.seed(1000 * seed + step)
-        (ot, ob), op_ = o.sample(n, unique=unique)
-        assert np.array_equal(rt, ot) and np.array_equal(rb, ob) and np.array_equal(rp, op_)
-        pri = (rng.random(len(rt)) + 0.01).astype(np.float32)
-        r.update_batch_priorities(pri)
-        o.update_batch_priorities(pri)
-        assert np.array_equal(r.tree, o.tree)
+    got = C.sum_tree_trace(SumTree, seed)
+    for k, x in got.items():
+        want = ref[f"sum_tree/{seed}/{k}"]
+        assert x.shape == want.shape and np.array_equal(x, want), k

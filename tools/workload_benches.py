@@ -1,6 +1,6 @@
 """bench.py --workload gae | replay | dqn: BASELINE.json configs[1] and configs[3] in the same line format as the
 PPO workload (metric/value/unit, e2e through the public API with HOST buffers, roofline of the dominant kernel
-against MEASURED_PEAKS.json, cpu_baseline = the unmodified reference from baseline/_ref on the host cores, or
+against MEASURED_PEAKS.json, cpu_baseline = the unmodified reference from oracle/_ref on the host cores, or
 the oracle port when it is absent).  The driver only runs the default PPO workload; lines of these workloads
 measured on a B200 are kept under profiles/ (tools/run_workloads.sh).
 
